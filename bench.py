@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 1|4|5]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 1|4|5] [--dump-outputs DIR]
 
 Workloads (config.workload names the one that ran):
   --config 1 (default): configs[1] = "xz -6 bt4, 8 MiB dict, 1 GiB synthetic text, 64 .xz blocks" (16 MiB
@@ -182,6 +182,25 @@ def block_hashes(buf, recs):
     return out
 
 
+DUMP_SAMPLE = 8 * MiB  # encoded bytes kept by --dump-outputs (32 MB as float32)
+
+
+def dump_outputs(out_dir, blocks, recs):
+    """What the timed encode returned in its last step, as arrays two builds can be compared with:
+    index_records.npy  (unpadded size, uncompressed size) of every Block, float64 (exact below 2**53);
+    block_sha256.npy   SHA-256 of every Block, one row of 32 bytes per Block, float32;
+    blocks_sample.npy  the encoded bytes at DUMP_SAMPLE positions drawn with a fixed seed (all bytes when
+                       there are fewer), float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "index_records.npy"), np.array(recs, dtype=np.float64).reshape(-1, 2))
+    sha = [np.frombuffer(bytes.fromhex(h), dtype=np.uint8) for _, h in block_hashes(blocks.tobytes(), recs)]
+    np.save(os.path.join(out_dir, "block_sha256.npy"), np.array(sha, dtype=np.float32).reshape(-1, 32))
+    if len(blocks) > DUMP_SAMPLE:
+        blocks = blocks[np.sort(np.random.default_rng(0).integers(0, len(blocks), DUMP_SAMPLE))]
+    np.save(os.path.join(out_dir, "blocks_sample.npy"), blocks.astype(np.float32))
+
+
 def run_reference(args):
     """Reference arm: lzma_stream_encoder_mt of the unmodified reference on the host cores."""
     import xzlibs as X
@@ -340,6 +359,8 @@ def run_ours(args):
                 stat_acc[k] = stat_acc.get(k, 0) + v
     clocks = sampler.stop() if rank == 0 else None
     n_steps = len(dev_times)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, h_out[:size_h].numpy(), recs)
 
     # ---- parity: every Block of this rank against the reference's golden vectors ----
     mine = h_out[:size_h].numpy().tobytes()
@@ -487,6 +508,8 @@ def main():
     ap.add_argument("--ref-blocks", type=int, default=0, help="--impl reference: Blocks per step (0 = automatic bound)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-lzma-code", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write rank 0's output of the last timed step to DIR/*.npy (records, per-Block SHA-256, seeded byte sample)")
     ap.add_argument("--scaling", default=None, choices=["weak", "strong"],
                     help="N > 1: weak = the config's job per GPU (default for --config 1), strong = the config's job split over the GPUs")
     args = ap.parse_args()

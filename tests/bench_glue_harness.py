@@ -1,7 +1,7 @@
 """CPU dry run of bench.py's host glue (argument handling, Block sharding, the Index record gather, the
 JSON line) for tests/test_bench_glue_cpu.py: torch.cuda and the GPU context are replaced by stand-ins --
-the stand-in context encodes with the unmodified reference (oracle/_ref), so the run needs no GPU and says
-nothing about the product path.  Launched under torch.distributed.run with the gloo backend."""
+the stand-in context encodes with the oracle (oracle/liboracle.so, the CPU restatement of the reference), so the
+run needs no GPU and says nothing about the product path.  Launched under torch.distributed.run with the gloo backend."""
 import ctypes as C
 import os
 import sys
@@ -28,7 +28,7 @@ def _vli(b, pos):
 
 
 class FakeContext:
-    """Same method names and return shapes as xz_b200.Context; Blocks come from the reference on the CPU."""
+    """Same method names and return shapes as xz_b200.Context; Blocks come from the oracle on the CPU."""
 
     def __init__(self, device=0):
         self._stats = {}
@@ -51,7 +51,7 @@ class FakeContext:
         for off in range(0, n, block_size):
             blk = data[off:off + block_size]
             buf = (C.c_uint8 * len(blk)).from_buffer_copy(blk)
-            xz = X.ref_encode(buf, len(blk), 0, block_size, threads=1, opts=opts)
+            xz = X.oracle_encode(buf, len(blk), 0, block_size, opts=opts)
             index_size = (int.from_bytes(xz[-8:-4], "little") + 1) * 4
             body = xz[12:len(xz) - 12 - index_size]
             idx = xz[len(xz) - 12 - index_size:]
@@ -71,7 +71,7 @@ class FakeContext:
 
     def stream_decode_into(self, src, n, dst, cap):
         t0 = time.perf_counter()
-        r, out = X.ref_decode(C.string_at(src, n), cap)
+        r, out = X.oracle_decode(C.string_at(src, n), cap)
         C.memmove(dst, out, len(out))
         ms = (time.perf_counter() - t0) * 1e3
         self._stats = {"ms_total": ms, "ms_h2d": 0.0, "ms_d2h": 0.0}

@@ -13,10 +13,12 @@
    records sizes, SHA-256 and return codes in buffer_golden.json.
 5. (`make_golden.py trace`) records the reference's lzma_code() return-code sequences
    (LZMA_TELL_* / LZMA_CONCATENATED / LZMA_IGNORE_CHECK flags) for the corpus in stream_trace_golden.json.
+6. (`make_golden.py live <reference source tree>`) records what the tests compare with the reference on their own
+   inputs (ref_checks_golden.json, ref_xz_*.xz), so that they need neither the reference nor oracle/_ref.
 3. Stores the reference's known-answer values for CRC32/CRC64 (tests/test_check.c:74,112) and the
    MicroLZMA encoder KAT (tests/test_microlzma.c:20-32) in kat.json.
 """
-import glob, hashlib, json, os, shutil, sys
+import glob, hashlib, json, os, re, shutil, sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
@@ -159,6 +161,110 @@ def trace_inputs():
             "gen:none+garbage": a + b"garbage!"}
 
 
+def main_live(ref_tree):
+    """What the tests compare with the reference on their own inputs, recorded once so that they run without it:
+    ref_checks_golden.json (sizes + SHA-256 of the reference's output, its return codes, struct layouts and symbol
+    tables) and two single-threaded `xz -6 -T1` Streams (Blocks without sizes) as ref_xz_*.xz."""
+    import ctypes as C
+    import random
+    import subprocess
+    import tempfile
+    assert X.have_ref(), "build oracle/_ref first (make -f oracle/Makefile.ref all)"
+    sys.path.insert(0, X.ROOT)
+    import test_api_cpu as API
+    import test_filters_cpu as FC
+    import test_gpu_filters as GF
+    MiB, KiB = 1 << 20, 1 << 10
+    g = {}
+    # tests/test_oracle.py
+    g["buffer_encode"] = {f"{kind}|{preset:#x}|{n}|{check}": X.digest(X.ref_buffer_encode(X.gendata(kind, n), n, preset, check))
+                          for kind, preset, n in (("T", 6, 1234567), ("E", 9 | X.XZ_PRESET_EXTREME, 200001), ("R", 1, 131072), ("L", 3, 700000))
+                          for check in (0, 1, 4)}
+    g["stream_encode"] = {}
+    for kind in "TER":
+        for preset, n, bs in ((1, 1 * MiB + 3, 512 * 1024), (6, 600001, 256 * 1024), (3, 700000, 1 * MiB)):
+            buf = X.gendata(kind, n)
+            xz = X.ref_encode(buf, n, preset, bs)
+            r, out = X.ref_decode(xz, n)
+            rm, outm = X.ref_decode(xz, n, mt=True)
+            g["stream_encode"][f"{kind}|{preset}|{n}|{bs}"] = {"xz": X.digest(xz), "decode": [r] + X.digest(out), "decode_mt": [rm] + X.digest(outm)}
+    buf = X.gendata("T", 300000)
+    g["match_finders"] = {}
+    for mode in (1, 2):
+        for mf in (0x03, 0x04, 0x12, 0x13, 0x14):
+            for lc, lp, pb in ((3, 0, 2), (0, 2, 0), (4, 0, 4), (1, 3, 1)):
+                o = X.LzmaOptions(1 << 20, lc, lp, pb, mode, 32, mf, 0)
+                g["match_finders"][f"{mode}|{mf:#x}|{lc}|{lp}|{pb}"] = X.digest(X.ref_encode(buf, 300000, 0, 1 << 20, opts=o))
+    xz = X.ref_encode(X.gendata("T", 50000), 50000, 6, 1 << 16)
+    bad = bytearray(xz)
+    bad[len(xz) // 2] ^= 0x55
+    g["truncated"] = {"xz": X.digest(xz), "cut": {str(cut): X.ref_decode(xz[:cut], 50000)[0] for cut in (5, 40, len(xz) // 2, len(xz) - 1)},
+                      "flipped": X.ref_decode(bytes(bad), 50000)[0]}
+    # tests/test_api_cpu.py
+    with tempfile.TemporaryDirectory() as d:
+        src, exe = os.path.join(d, "l.c"), os.path.join(d, "l")
+        open(src, "w").write(API.LAYOUT_PROG.replace("HEADER", "<lzma.h>"))
+        subprocess.check_call(["gcc", "-I", os.path.join(ref_tree, "src", "liblzma", "api"), src, "-o", exe])
+        g["lzma_h_layout"] = subprocess.check_output([exe], text=True)
+    ref = C.CDLL(os.path.join(X.ROOT, "oracle", "_ref", "liblzma_ref.so"))
+    ref.lzma_mt_block_size.restype = C.c_uint64
+    g["mt_options"] = {}
+    for kw, _ in API.BAD_OPTIONS:
+        s = API.LzmaStream()
+        g["mt_options"][json.dumps(kw, sort_keys=True)] = ref.lzma_stream_encoder_mt(C.byref(s), C.byref(API._mt(**kw)))
+        ref.lzma_end(C.byref(s))
+    g["filter_chains"] = {}
+    for spec in API.BAD_CHAINS + API.GOOD_CHAINS:
+        keep = []
+        arr = API._chain(spec, keep)
+        s = API.LzmaStream()
+        r = ref.lzma_stream_encoder_mt(C.byref(s), C.byref(API._mt(filters=C.cast(arr, C.c_void_p))))
+        ref.lzma_end(C.byref(s))
+        g["filter_chains"][API.chain_id(spec)] = {"ret": r, "mt_block_size": ref.lzma_mt_block_size(arr) if r == 0 else None}
+    # tests/test_filters_cpu.py
+    g["bcj"] = {}
+    for fid, arg in FC.BCJ_CASES:
+        for n in FC.BCJ_SIZES:
+            data = FC.codeish(fid, n, 1000 * fid + n)
+            g["bcj"][f"{fid}|{arg}|{n}"] = [hashlib.sha256(X.ref_filter_apply(fid, arg, e, data)).hexdigest() for e in (1, 0)]
+    g["delta"] = {}
+    for dist in FC.DELTA_DISTS:
+        for n in FC.DELTA_SIZES:
+            rnd = random.Random(dist * 7 + n)
+            data = bytes(rnd.getrandbits(8) for _ in range(n))
+            g["delta"][f"{dist}|{n}"] = [hashlib.sha256(X.ref_filter_apply(FC.DELTA, dist, e, data)).hexdigest() for e in (1, 0)]
+    # tests/test_gpu_filters.py
+    data = GF.mixed_input(700 * KiB + 123, 17)
+    g["chain_encode"] = {API.chain_id(chain): X.digest(X.ref_chain_encode(data, chain, 6, 256 * KiB)) for chain in GF.CHAINS}
+    rnd = random.Random(5)
+    data = bytes(rnd.getrandbits(8) for _ in range(300 * KiB))
+    g["chain_encode_random"] = {f"{preset}|{API.chain_id(chain)}": X.digest(X.ref_chain_encode(data, chain, preset, 128 * KiB))
+                                for preset in (0, 3) for chain in GF.RANDOM_CHAINS}
+    # tests/test_gpu_lzma_api.py
+    a, b = X.gendata("T", 100000), X.gendata("E", 70000)
+    xa, xb = X.ref_encode(a, 100000, 6, 1 << 16), X.ref_encode(b, 70000, 1, 1 << 15)
+    g["concat_pad"] = {"inputs": [X.digest(xa), X.digest(xb)]}
+    for pad in (0, 8, 6):
+        cat = xa + b"\0" * pad + xb
+        o2 = (C.c_uint8 * 200000)(); s2 = C.c_size_t()
+        g["concat_pad"][str(pad)] = X.ref().ref_decode_flags(cat, C.c_size_t(len(cat)), C.c_uint32(0x08), o2, C.c_size_t(200000), C.byref(s2))
+    n = 3 * MiB + 17
+    xz = X.ref_buffer_encode(X.gendata("E", n), n, 2, 4)
+    r, back, used = X.ref_buffer_decode(xz, n)
+    g["buffer_roundtrip"] = {"xz": X.digest(xz), "decode": [r, used] + X.digest(back)}
+    xz_cli = os.path.join(X.ROOT, "oracle", "_ref", "xz")
+    for name, data in (("T6_300000", bytes(X.gendata("T", 300000)[:300000])), ("zeros_40000000", bytes(40 * 1000 * 1000))):
+        st = subprocess.run([xz_cli, "-6", "-T1"], input=data, stdout=subprocess.PIPE, check=True).stdout
+        open(os.path.join(HERE, f"ref_xz_{name}_T1.xz"), "wb").write(st)
+    # tests/test_hybrid_cpu.py: the lzma_* symbols the reference `xz` imports and the ones the reference liblzma defines
+    def syms(path, flag):
+        out = subprocess.run(["nm", "-D", flag, path], stdout=subprocess.PIPE, text=True, check=True).stdout
+        return sorted({ln.split()[-1] for ln in out.splitlines() if re.search(r"\blzma_", ln)})
+    g["xz_imports"] = syms(xz_cli, "--undefined-only")
+    g["ref_liblzma_exports"] = syms(os.path.join(X.ROOT, "oracle", "_ref", "liblzma_ref.so"), "--defined-only")
+    json.dump(g, open(os.path.join(HERE, "ref_checks_golden.json"), "w"), indent=0, sort_keys=True)
+
+
 def main():
     assert X.have_ref(), "build oracle/_ref first (make -f oracle/Makefile.ref all)"
     dst = os.path.join(HERE, "ref_files")
@@ -214,5 +320,7 @@ if __name__ == "__main__":
         main_buffer()
     elif len(sys.argv) > 1 and sys.argv[1] == "trace":
         main_trace()
+    elif len(sys.argv) > 2 and sys.argv[1] == "live":
+        main_live(sys.argv[2])
     else:
         main()

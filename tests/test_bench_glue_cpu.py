@@ -1,21 +1,15 @@
-"""bench.py's host glue at world sizes 1 and 2 without a GPU (tests/bench_glue_harness.py puts a reference-backed
+"""bench.py's host glue at world sizes 1 and 2 without a GPU (tests/bench_glue_harness.py puts an oracle-backed
 stand-in where the GPU context is): the sharding of the job, the record gather, the printed JSON line.  The numbers
-it prints are the reference's on the CPU and mean nothing; the shape of the line and the job arithmetic are the test."""
+it prints are the oracle's on the CPU and mean nothing; the shape of the line and the job arithmetic are the test."""
 import json
 import os
 import socket
 import subprocess
 import sys
 
-import pytest
-
-import xzlibs as X
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HARNESS = os.path.join(ROOT, "tests", "bench_glue_harness.py")
 MiB = 1 << 20
-
-pytestmark = pytest.mark.skipif(not X.have_ref(), reason="oracle/_ref not built")
 
 
 def _port():
@@ -48,6 +42,24 @@ def test_one_gpu_line():
     assert "decode(encode(x)) == x for every Block" in ln["parity"]
     for k in ("metric", "value", "unit", "ms_per_step", "higher_is_better", "scaling", "dtype", "data", "roofline", "clocks", "gpu_launches"):
         assert k in ln
+
+
+def test_dump_outputs(tmp_path):
+    """--dump-outputs: the last timed step's Index records, per-Block SHA-256 and encoded bytes, as float arrays."""
+    import hashlib
+    import numpy as np
+    _run(1, ["--dump-outputs", str(tmp_path)])
+    recs = np.load(tmp_path / "index_records.npy")
+    sha = np.load(tmp_path / "block_sha256.npy")
+    blocks = np.load(tmp_path / "blocks_sample.npy")
+    assert recs.dtype == np.float64 and recs.shape == (4, 2) and (recs[:, 1] == MiB).all()
+    assert sha.dtype == np.float32 and sha.shape == (4, 32) and blocks.dtype == np.float32
+    sizes = (recs[:, 0].astype(np.int64) + 3) // 4 * 4
+    assert len(blocks) == sizes.sum()   # 4 MiB of input: all encoded bytes, no sample
+    raw = blocks.astype(np.uint8).tobytes()
+    offs = np.concatenate([[0], np.cumsum(sizes)])
+    for i in range(4):
+        assert hashlib.sha256(raw[offs[i]:offs[i + 1]]).digest() == sha[i].astype(np.uint8).tobytes()
 
 
 def test_two_ranks_weak_scaling_job_is_per_gpu():

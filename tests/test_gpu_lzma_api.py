@@ -124,16 +124,14 @@ def test_lzma_code_sequence_rules(lib):
     lib.lzma_end(C.byref(s2))
 
 
-@pytest.mark.skipif(not X.have_ref(), reason="oracle/_ref not built")
 def test_decoder_finishes_unsized_stream_under_lzma_run_only(lib):
     """Callers that never pass LZMA_FINISH (Python's lzma module, libarchive): the reference's decoder returns
     LZMA_STREAM_END under LZMA_RUN once the Stream Footer is in (stream_decoder.c:309-331).  Single-threaded encoders
     write Blocks without sizes, so the end of the Stream is only found by decoding; here the input arrives in 8 KiB
-    pieces with LZMA_RUN throughout.  Also a ratio far above 64 : 1 (zeros), where the first output guess is too small."""
-    import subprocess
-    xz = os.path.join(X.ROOT, "oracle", "_ref", "xz")
-    for data in (bytes(X.gendata("T", 300000)[:300000]), bytes(40 * 1000 * 1000)):
-        comp = subprocess.run([xz, "-6", "-T1"], input=data, stdout=subprocess.PIPE, check=True).stdout
+    pieces with LZMA_RUN throughout.  Also a ratio far above 64 : 1 (zeros), where the first output guess is too small.
+    The Streams are the reference's `xz -6 -T1` output for these inputs (tests/golden/ref_xz_*_T1.xz)."""
+    for name, data in (("T6_300000", bytes(X.gendata("T", 300000)[:300000])), ("zeros_40000000", bytes(40 * 1000 * 1000))):
+        comp = open(os.path.join(GOLD, f"ref_xz_{name}_T1.xz"), "rb").read()
         d = LzmaStream()
         assert lib.lzma_stream_decoder(C.byref(d), C.c_uint64((1 << 64) - 1), C.c_uint32(0)) == 0
         ret, back = _drive(lib, d, comp, 8192, 1 << 20, final_action=RUN)
@@ -184,6 +182,7 @@ def test_concatenated_streams_and_padding(lib):
             assert hashlib.sha256(out).hexdigest() == v["out_concat_sha256"], name
     a, b = X.gendata("T", 100000), X.gendata("E", 70000)
     xa, xb = X.oracle_encode(a, 100000, 6, 1 << 16), X.oracle_encode(b, 70000, 1, 1 << 15)
+    assert [X.digest(xa), X.digest(xb)] == X.ref_golden()["concat_pad"]["inputs"]
     for pad, ok in ((0, True), (8, True), (6, False)):
         d = LzmaStream()
         assert lib.lzma_stream_decoder(C.byref(d), C.c_uint64((1 << 64) - 1), C.c_uint32(0x08)) == 0
@@ -193,11 +192,7 @@ def test_concatenated_streams_and_padding(lib):
             assert ret == 1 and out == bytes(a[:100000]) + bytes(b[:70000])
         else:
             assert ret == 9
-        if X.have_ref():
-            o2 = (C.c_uint8 * 200000)(); s2 = C.c_size_t()
-            data = xa + b"\0" * pad + xb
-            r2 = X.ref().ref_decode_flags(data, C.c_size_t(len(data)), C.c_uint32(0x08), o2, C.c_size_t(200000), C.byref(s2))
-            assert (r2 == 0) == ok
+        assert (X.ref_golden()["concat_pad"][str(pad)] == 0) == ok   # the reference's verdict on the same bytes
 
 
 # ---- one-shot buffer API: lzma_easy_buffer_encode / lzma_stream_buffer_encode / lzma_stream_buffer_decode ----
@@ -292,15 +287,14 @@ def test_stream_buffer_decode_matches_reference_verdicts(lib, name, kind, preset
 
 
 def test_buffer_roundtrip_through_reference_decoder(lib):
-    """Cross-check in the other direction where oracle/_ref travelled: the reference decodes our one-shot Stream."""
-    if not X.have_ref():
-        pytest.skip("oracle/_ref not present")
+    """Cross-check in the other direction: our one-shot Stream is the reference's, and the reference's
+    lzma_stream_buffer_decode gave the input back from it (tests/golden/ref_checks_golden.json)."""
     n = 3 * (1 << 20) + 17
     buf = X.gendata("E", n)
     r, xz, _ = _easy_buffer_encode(lib, buf, n, 2, 4)
-    assert r == 0 and xz == X.ref_buffer_encode(buf, n, 2, 4)
-    rr, back, used = X.ref_buffer_decode(xz, n)
-    assert rr == 0 and used == len(xz) and back == bytes(buf[:n])
+    ref = X.ref_golden()["buffer_roundtrip"]
+    assert r == 0 and X.digest(xz) == ref["xz"]
+    assert ref["decode"] == [0, len(xz)] + X.digest(bytes(buf[:n]))
 
 
 # ---- return-code sequences of the streaming decoder (LZMA_TELL_*, LZMA_CONCATENATED, LZMA_IGNORE_CHECK) ----

@@ -1,6 +1,6 @@
 """CPU tests (-m "not gpu"): pin the oracle (oracle/liboracle.so) against
   * the reference's own golden vectors / KATs / decoder corpus (tests/golden/), and
-  * the unmodified reference library (oracle/_ref) when it is present (build container).
+  * what the unmodified reference produced on the same inputs (tests/golden/ref_checks_golden.json).
 """
 import ctypes as C
 import glob
@@ -71,12 +71,12 @@ def test_oracle_buffer_encoder_matches_reference_golden(case):
     assert len(out) == case["xz_size"] and hashlib.sha256(out).hexdigest() == case["xz_sha256"]
 
 
-@pytest.mark.skipif(not X.have_ref(), reason="oracle/_ref not built")
 def test_oracle_buffer_encoder_vs_live_reference():
+    gold = X.ref_golden()["buffer_encode"]
     for kind, preset, n in (("T", 6, 1234567), ("E", 9 | X.XZ_PRESET_EXTREME, 200001), ("R", 1, 131072), ("L", 3, 700000)):
         buf = X.gendata(kind, n)
         for check in (0, 1, 4):
-            assert X.oracle_buffer_encode(buf, n, preset, check) == X.ref_buffer_encode(buf, n, preset, check)
+            assert X.digest(X.oracle_buffer_encode(buf, n, preset, check)) == gold[f"{kind}|{preset:#x}|{n}|{check}"]
 
 
 def test_oracle_encoder_config0_full_size():
@@ -107,29 +107,27 @@ def test_decoder_corpus_verdicts():
     assert n > 50
 
 
-@pytest.mark.skipif(not X.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("kind", "TER")
 def test_oracle_vs_live_reference(kind):
-    """Same run, same buffers: oracle restatement == unmodified reference, encode and decode."""
+    """Same inputs: oracle restatement == unmodified reference, encode, and the reference's decoders (single- and
+    multi-threaded) give the input back from that Stream."""
     for preset, n, bs in ((1, 1 * MiB + 3, 512 * 1024), (6, 600001, 256 * 1024), (3, 700000, 1 * MiB)):
         buf = X.gendata(kind, n)
         a = X.oracle_encode(buf, n, preset, bs)
-        b = X.ref_encode(buf, n, preset, bs)
-        assert a == b
-        r, out = X.ref_decode(a, n)
-        assert r == 0 and out == bytes(buf[:n])
-        r, out = X.ref_decode(a, n, mt=True)
-        assert r == 0 and out == bytes(buf[:n])
+        ref = X.ref_golden()["stream_encode"][f"{kind}|{preset}|{n}|{bs}"]
+        assert X.digest(a) == ref["xz"]
+        want = [0] + X.digest(bytes(buf[:n]))
+        assert ref["decode"] == want and ref["decode_mt"] == want
 
 
-@pytest.mark.skipif(not X.have_ref(), reason="oracle/_ref not built")
 def test_oracle_vs_live_reference_all_match_finders():
     buf = X.gendata("T", 300000)
+    gold = X.ref_golden()["match_finders"]
     for mode in (1, 2):
         for mf in (0x03, 0x04, 0x12, 0x13, 0x14):
             for lc, lp, pb in ((3, 0, 2), (0, 2, 0), (4, 0, 4), (1, 3, 1)):
                 o = X.LzmaOptions(1 << 20, lc, lp, pb, mode, 32, mf, 0)
-                assert X.oracle_encode(buf, 300000, 0, 1 << 20, opts=o) == X.ref_encode(buf, 300000, 0, 1 << 20, opts=o)
+                assert X.digest(X.oracle_encode(buf, 300000, 0, 1 << 20, opts=o)) == gold[f"{mode}|{mf:#x}|{lc}|{lp}|{pb}"]
 
 
 def test_truncated_and_corrupt_streams():
@@ -142,7 +140,8 @@ def test_truncated_and_corrupt_streams():
     bad[len(xz) // 2] ^= 0x55
     r, _ = X.oracle_decode(bytes(bad), 50000)
     assert r == 9
-    if X.have_ref():
-        for cut in (5, 40, len(xz) // 2, len(xz) - 1):
-            assert X.ref_decode(xz[:cut], 50000)[0] == 10
-        assert X.ref_decode(bytes(bad), 50000)[0] == 9
+    ref = X.ref_golden()["truncated"]
+    assert X.digest(xz) == ref["xz"]
+    for cut in (5, 40, len(xz) // 2, len(xz) - 1):
+        assert ref["cut"][str(cut)] == 10
+    assert ref["flipped"] == 9

@@ -1,6 +1,8 @@
 """ctypes bindings used by the tests: the oracle (checker), oracle/_ref (the unmodified
 reference, when built), the input generator, and the product C-ABI library."""
 import ctypes as C
+import hashlib
+import json
 import os
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -149,6 +151,43 @@ def ref_encode(buf, n, preset, block_size, check=CHECK_CRC64, threads=0, opts=No
                                      C.c_size_t(cap), C.byref(sz))
     assert r == 0, r
     return bytes(out[:sz.value])
+
+
+def ref_filter_apply(fid, arg, enc, data):
+    """One Delta / BCJ filter of the unmodified reference over `data` (encoder direction when enc)."""
+    n = len(data)
+    out = (C.c_uint8 * n)()
+    ids = (C.c_uint32 * 1)(fid); args = (C.c_uint32 * 1)(arg)
+    r = ref().ref_filter_apply(ids, args, C.c_uint32(1), C.c_int(enc), bytes(data), C.c_size_t(n), out)
+    assert r == 0, r
+    return bytes(out)
+
+
+def ref_chain_encode(data, chain, preset, bs, check=CHECK_CRC64):
+    """lzma_stream_encoder_mt of the unmodified reference with the filter chain [(id, arg), ...] in front of LZMA2."""
+    n = len(data)
+    cap = n + n // 2 + 65536
+    out = (C.c_uint8 * cap)()
+    sz = C.c_size_t()
+    ids = (C.c_uint32 * len(chain))(*[c[0] for c in chain])
+    args = (C.c_uint32 * len(chain))(*[c[1] for c in chain])
+    r = ref().ref_encode_mt_chain(data, C.c_size_t(n), ids, args, C.c_uint32(len(chain)), C.c_uint32(preset), C.c_uint64(bs), C.c_uint32(check),
+                                  C.c_uint32(4), out, C.c_size_t(cap), C.byref(sz))
+    assert r == 0, r
+    return bytes(out[:sz.value])
+
+
+def ref_golden():
+    """What the tests compare with the reference on their own inputs (tests/golden/make_golden.py live)."""
+    if "golden" not in _cache:
+        with open(os.path.join(ROOT, "tests", "golden", "ref_checks_golden.json")) as f:
+            _cache["golden"] = json.load(f)
+    return _cache["golden"]
+
+
+def digest(b):
+    """[size, SHA-256] as ref_checks_golden.json stores the reference's output."""
+    return [len(b), hashlib.sha256(b).hexdigest()]
 
 
 def ref_decode(data, cap, mt=False):
